@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # ours (CUDA engine through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm's CPU path (C port)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed result to DIR/msm_result.npy
 
 A "step" is one bn254 G1 MultiExp over one batch of synthetic inputs.  Metric: scalar-muls/s = n_total / time.
   N = 1   BASELINE.json configs[1]: n = 2^24, window width from the engine's model.
@@ -454,6 +455,15 @@ def fail_parity(what, res):
         raise SystemExit("bench.py: PARITY FAILURE (%s): the timed result differs from the closed form" % what)
 
 
+def dump_outputs(out_dir, result_jac):
+    """--dump-outputs: the headline's last timed result, the Jacobian triple (X, Y, Z) of Montgomery limbs the engine returns,
+    as msm_result.npy: one row per coordinate, each u64 limb split into its two u32 halves (low half first) so that float64
+    holds every word exactly"""
+    os.makedirs(out_dir, exist_ok=True)
+    words = np.ascontiguousarray(result_jac, dtype=np.uint64).view(np.uint32).reshape(3, -1)
+    np.save(os.path.join(out_dir, "msm_result.npy"), words.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -473,7 +483,12 @@ def main():
     ap.add_argument("--no-tables", action="store_true", help="skip the window-table (precomputed resident bases) measurement")
     ap.add_argument("--no-extras", action="store_true", help="skip the sub-objects (configs[2], [3], 2^20, 2^26, skewed scalars, concurrent calls)")
     ap.add_argument("--table-c", type=int, default=0, help="window width of the table mode (0 = engine model)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the headline's last timed step to DIR/msm_result.npy (float64), to compare two builds "
+                         "output for output (the inputs are fixed by their seeds)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -529,6 +544,8 @@ def main():
 
     res, K = measure_resident(X, g, logn_local, args.steps, args.warmup, c=args.c, sample_clocks=True)
     fail_parity("headline", res)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, K.result_jac)
     line = {
         "metric": metric_name(g),
         "value": res["value"], "unit": "scalar-muls/s", "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
