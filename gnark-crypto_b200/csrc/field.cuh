@@ -161,6 +161,15 @@ GMSM_HD uint32_t modm(int j) {
   return P::mod(j);
 }
 
+// k * q < 2^(32N), evaluated at compile time from the modulus limbs: the bound the fused multi-product reductions need for
+// their intermediate frames (fp_dot4: frames below 5q)
+template <class P>
+GMSM_HD constexpr bool mod_multiple_fits(uint32_t k) {
+  uint64_t c = 0;
+  for (int i = 0; i < P::N; i++) c = ((uint64_t)P::mod(i) * k + (c >> 32));
+  return (c >> 32) == 0;
+}
+
 // r = (a >= q) ? a - q : a, for a value a + carry * 2^(32N) < 2q.  carry is always 0 for the moduli with a spare top bit
 // (2q < 2^(32N)); the full-width moduli (secp256k1 fp and fr, P::FULL) hand in the carry-out of the addition / the carry limb of
 // the multiplier: a - q then wraps to the right N limbs
@@ -647,6 +656,7 @@ template <class P>
 GMSM_HD Fp<P> fp_dot4_inline(const Fp<P>& x0, const Fp<P>& y0, const Fp<P>& x1, const Fp<P>& y1, const Fp<P>& x2, const Fp<P>& y2,
                              const Fp<P>& x3, const Fp<P>& y3) {
   constexpr int N = P::N;
+  static_assert(mod_multiple_fits<P>(5), "needs 5q < 2^(32N) (frames below 5q)");
   Fp<P> r;
   uint32_t A[N + 2], B[N + 2];
 #pragma unroll
@@ -764,7 +774,7 @@ template <class P>
 GMSM_HD Fp<P> fp_dot4(const Fp<P>& x0, const Fp<P>& y0, const Fp<P>& x1, const Fp<P>& y1, const Fp<P>& x2, const Fp<P>& y2,
                       const Fp<P>& x3, const Fp<P>& y3) {
 #if defined(GMSM_DOT4) && defined(GMSM_PTX_PATH) && !defined(GMSM_PORTABLE_MUL)
-  if constexpr ((P::mod(P::N - 1) >> 30) == 0) {
+  if constexpr (mod_multiple_fits<P>(5)) {   // bn254: 5q = 0.945 * 2^256; a q in [0.2, 0.25) * 2^(32N) takes two fp_dot2
 #if defined(__CUDA_ARCH__) && defined(GMSM_MUL_NOINLINE)
     return fp_dot4_ni<P>(x0, y0, x1, y1, x2, y2, x3, y3);
 #else
@@ -1112,5 +1122,9 @@ template <class P> GMSM_HD Fp<P> f_dot2(const Fp<P>& x, const Fp<P>& y, const Fp
 template <class P> GMSM_HD Fp<P> f_dbl(const Fp<P>& a) { return fp_dbl(a); }
 template <class P> GMSM_HD Fp<P> f_neg(const Fp<P>& a) { return fp_neg(a); }
 template <class P> GMSM_HD Fp<P> f_inv(const Fp<P>& a) { return fp_inv(a); }
+
+// the prime field a coordinate field is built on (Fp itself here; the Fp2 specialisation is in fp2.cuh)
+template <class F> struct base_field;
+template <class P> struct base_field<Fp<P>> { using type = Fp<P>; };
 
 }  // namespace gmsm

@@ -21,6 +21,8 @@ struct Fp2 {
   GMSM_HD bool operator!=(const Fp2& b) const { return !(*this == b); }
 };
 
+template <class P> struct base_field<Fp2<P>> { using type = Fp<P>; };
+
 template <class P> GMSM_HD Fp2<P> f_add(const Fp2<P>& a, const Fp2<P>& b) { return Fp2<P>{fp_add(a.a0, b.a0), fp_add(a.a1, b.a1)}; }
 template <class P> GMSM_HD Fp2<P> f_sub(const Fp2<P>& a, const Fp2<P>& b) { return Fp2<P>{fp_sub(a.a0, b.a0), fp_sub(a.a1, b.a1)}; }
 template <class P> GMSM_HD Fp2<P> f_dbl(const Fp2<P>& a) { return Fp2<P>{fp_dbl(a.a0), fp_dbl(a.a1)}; }

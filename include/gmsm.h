@@ -226,7 +226,9 @@ enum {
   GMSM_OP_ADD = 9,                         /* a: xyzz, b: xyzz -> xyzz */
   GMSM_OP_DOUBLE = 10,                     /* a: xyzz -> xyzz */
   GMSM_OP_TO_AFFINE = 11,                  /* a: xyzz -> affine */
-  GMSM_OP_FR_FROM_MONT = 12                /* a: scalar -> canonical scalar */
+  GMSM_OP_FR_FROM_MONT = 12,               /* a: scalar -> canonical scalar */
+  GMSM_OP_DOT2 = 13,                       /* a: [x | u], b: [y | v] -> x*y + u*v (coordinate field, fused form) */
+  GMSM_OP_FP_DOT4 = 14                     /* a: x0..x3, b: y0..y3 -> sum x_k*y_k (base field, fused form) */
 };
 int gmsm_test_op(gmsm_curve_t curve, int op, const uint32_t* a, const uint32_t* b, uint32_t* out,
                  size_t n);

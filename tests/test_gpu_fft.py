@@ -49,6 +49,46 @@ def test_fft_matches_oracle(curve, logn):
     d.close()
 
 
+def _edge_inputs(f, n):
+    """Fr vectors at the edges of the Montgomery arithmetic (plain values; _enc stores value * R mod q)"""
+    q = f.q
+    raw_qm1 = (q - 1) * f.Rinv % q                                  # stored limbs q - 1
+    return {
+        "all_q-1": [q - 1] * n,
+        "all_limbs_q-1": [raw_qm1] * n,
+        "alternating_0_q-1": [0 if i % 2 == 0 else q - 1 for i in range(n)],
+        "alternating_limbs": [raw_qm1 if i % 2 == 0 else 0 for i in range(n)],
+        "powers_of_two": [(1 << (i % f.bits)) % q for i in range(n)],
+    }
+
+
+@pytest.mark.parametrize("curve", ["bn254", "bls12381", "bls12377"])
+@pytest.mark.parametrize("logn", [10, 11, 14])
+def test_fft_edge_inputs(curve, logn):
+    """extreme Fr inputs through the device FFT at one tile (2^10), one global stage (2^11) and four global stages (2^14):
+    FFT and FFTInverse, DIT and DIF, plain and on the coset, in full against the oracle; then the same on a domain whose
+    coset shift is q - 1"""
+    fft = _fft()
+    f = O.FIELDS[FR[curve]]
+    n = 1 << logn
+    od = O.FFTDomain(FR[curve], n)
+    d = fft.NewDomain(curve, n)
+    od_m1 = O.FFTDomain(FR[curve], n, shift=f.q - 1)
+    d_m1 = fft.NewDomain(curve, n, shift=_enc(f, [f.q - 1])[0])
+    try:
+        for name, vals in _edge_inputs(f, n).items():
+            for dec in (O.DIT, O.DIF):
+                for coset in (False, True):
+                    assert _dec(f, d.FFT(_enc(f, vals), dec, OnCoset=coset)) == od.fft(vals, dec, coset), (name, dec, coset)
+                    assert _dec(f, d.FFTInverse(_enc(f, vals), dec, OnCoset=coset)) == od.fft_inverse(vals, dec, coset), (name, dec, coset)
+                if name in ("all_q-1", "alternating_0_q-1"):
+                    assert _dec(f, d_m1.FFT(_enc(f, vals), dec, OnCoset=True)) == od_m1.fft(vals, dec, True), (name, dec, "shift q-1")
+                    assert _dec(f, d_m1.FFTInverse(_enc(f, vals), dec, OnCoset=True)) == od_m1.fft_inverse(vals, dec, True), (name, dec, "shift q-1")
+    finally:
+        d.close()
+        d_m1.close()
+
+
 def test_fft_custom_shift_and_errors():
     fft = _fft()
     f = O.FIELDS["bn254_fr"]

@@ -1,7 +1,7 @@
 """CPU builds (g++) of the product's field / curve headers against the oracle, without a GPU, in two variants:
 "portable" = the plain C++ arithmetic path; "emulated" = the device's carry-chain formulation (the source ptxas sees,
 -DGMSM_EMULATE_PTX: mad.lo.cc / madc.hi.cc / addc ... over an emulated carry flag, dropped carries trap).  The PTX itself
-is checked by the same vectors on the GPU in tests/test_gpu_ops.py."""
+is checked by the same vectors on the GPU in tests/test_gpu_ops.py and tests/test_gpu_arith_edges.py."""
 import ctypes
 import os
 import subprocess
@@ -88,8 +88,16 @@ def test_field_ops_host(hc, g):
 
 
 @pytest.mark.parametrize("g", list(O.GROUPS))
+def test_field_edges_host(hc, g):
+    """extreme operands (opcases.extreme_values) through every coordinate-field op, the fused sums of two and four products
+    and the inversion, against big-integer arithmetic on the raw limbs: each variant's formulation of the carry chains"""
+    opcases.check_field_edges(O.GROUPS[g], _runner(hc, g), n_random=64, n_perm=3)
+
+
+@pytest.mark.parametrize("g", list(O.GROUPS))
 def test_point_ops_host(hc, g):
     opcases.check_point_ops(O.GROUPS[g], _runner(hc, g))
+    opcases.check_point_edges(O.GROUPS[g], _runner(hc, g))
 
 
 @pytest.mark.parametrize("g,c", [("bn254_g1", 5), ("bn254_g1", 22), ("bn254_g2", 7), ("bls12381_g1", 11), ("bls12381_g2", 3),
@@ -139,14 +147,7 @@ def test_carry_chain_mul_sqr_stress(g):
     nl = f.limbs * 2
     import random
     r = random.Random(5)
-    vals = [0, 1, 2, f.q - 1, f.q - 2, f.Rmod, f.R2, (f.q - 1) // 2, (f.q + 1) // 2]
-    for k in range(0, 32 * nl, 7):
-        vals += [(1 << k) % f.q, ((1 << k) - 1) % f.q, (f.q - (1 << k)) % f.q]
-    top = (1 << (32 * nl)) - 1
-    for k in range(nl):
-        vals.append((top ^ (0xFFFFFFFF << (32 * k))) % f.q)
-        vals.append((0xFFFFFFFF << (32 * k)) % f.q)
-    vals += [r.randrange(f.q) for _ in range(3000)]
+    vals = opcases.extreme_values(f) + [r.randrange(f.q) for _ in range(3000)]
     A = np.array([f.to_limbs(v) for v in vals], dtype=np.uint64).view(np.uint32).reshape(len(vals), nl)
     perm = rng.permutation(len(vals))
     B = A[perm]
