@@ -152,23 +152,34 @@ static double model_ms(int curve, int fr_bits, size_t n, int c) {
   const double e_ns = m.add_ns * (1.0 + 0.012 * std::max(0, c - 17)) + 0.009;
   return (double)n * p.nwin * e_ns * 1e-6 + tail;
 }
-static int choose_c_for(int curve, int fr_bits, size_t n) {
+// Entries (one per non-zero digit) are numbered with 32-bit indices: a context holds at most max_n * W < MAX_ENTRIES of them.
+// With K <= 256 this also keeps the end of the last accumulate chunk, start + K, below 2^32.
+static constexpr double MAX_ENTRIES = 4294967000.0;
+static bool entries_fit(int fr_bits, size_t capacity, int c) { return (double)capacity * make_plan(fr_bits, c).nwin < MAX_ENTRIES; }
+
+// n: the size the model prices; capacity: the largest n ONE context built with the width has to hold (a pipelined call's largest
+// batch, not its total).  Only widths whose capacity * W fits the entry index are candidates: [4, 22] first, then c = 23, 24
+// (from n ~ 3.6e8 on the 253..256-bit fields no width up to 22 fits, c = 24 with W = 11 does).  When no width fits, the model's
+// unconstrained choice is returned and ctx_create_ex refuses it with the 32-bit-index error.
+static int choose_c_for(int curve, int fr_bits, size_t n, size_t capacity) {
   if (const char* e = getenv("GMSM_C")) {
     int c = atoi(e);
     if (c >= 2 && c <= 24) return c;
   }
-  double best = 1e300;
-  int bc = 13;
-  for (int c = 4; c <= 22; c++) {
-    const double t = model_ms(curve, fr_bits, n, c);
-    if (t < best) { best = t; bc = c; }
-  }
-  return bc;
+  auto best_of = [&](int lo, int hi, bool must_fit) {
+    double best = 1e300;
+    int bc = 0;
+    for (int c = lo; c <= hi; c++) {
+      if (must_fit && !entries_fit(fr_bits, capacity, c)) continue;
+      const double t = model_ms(curve, fr_bits, n, c);
+      if (t < best) { best = t; bc = c; }
+    }
+    return bc;
+  };
+  if (int c = best_of(4, 22, true)) return c;
+  if (int c = best_of(23, 24, true)) return c;
+  return best_of(4, 22, false);
 }
-static int curve_of_bits_default(int fr_bits) {
-  return fr_bits == 254 ? GMSM_BN254_G1 : fr_bits == 255 ? GMSM_BLS12381_G1 : fr_bits == 256 ? GMSM_SECP256K1_G1 : fr_bits == 377 ? GMSM_BW6761_G1 : fr_bits == 315 ? GMSM_BW6633_G1 : GMSM_BLS12377_G1;
-}
-static int choose_c(int fr_bits, size_t n) { return choose_c_for(curve_of_bits_default(fr_bits), fr_bits, n); }
 
 // window width of the window-table mode: one shared bucket set, so the bucket reduction costs 2^(c-1) * ~3.8
 // full-add equivalents ONCE instead of per window, and c can grow until that term meets the W(c)*n accumulate
@@ -314,7 +325,7 @@ static gmsm_ctx* ctx_create_ex(gmsm_curve_t curve, size_t max_n, int c, int devi
   ctx->device = device;
   ctx->max_n = max_n;
   ctx->ci = ci;
-  if (c == 0) c = shared ? choose_c_tables(ci.fr_bits, max_n) : choose_c_for(curve, ci.fr_bits, max_n);
+  if (c == 0) c = shared ? choose_c_tables(ci.fr_bits, max_n) : choose_c_for(curve, ci.fr_bits, max_n, max_n);
   ctx->shared = shared;
   // bucket accumulation: extended-Jacobian segmented reduction by default (INT-multiplier bound at 89 % of the
   // pipe); GMSM_AFFINE=1 selects the batch-affine tree (fewer multiplies, but 3x the HBM traffic: measured
@@ -337,7 +348,7 @@ static gmsm_ctx* ctx_create_ex(gmsm_curve_t curve, size_t max_n, int c, int devi
   if (const char* e = getenv("GMSM_SPLIT_W")) { int v = atoi(e); if (v >= 1 && v <= 64) ctx->split_w = ctx->split_tab = v; }
   ctx->plan = make_plan(ci.fr_bits, c);
   if (shared) ctx->plan.nb_total = std::max(ctx->plan.nb, ctx->plan.nb_last);   // one bucket set for all windows
-  if ((double)max_n * ctx->plan.nwin >= 4294967000.0) {
+  if ((double)max_n * ctx->plan.nwin >= MAX_ENTRIES) {
     set_err(GMSM_EINVAL, "n*W = %zu*%d does not fit the 32-bit entry index; shard the MSM", max_n, ctx->plan.nwin);
     l2_granularity_release(device);
     delete ctx;
@@ -675,27 +686,18 @@ static void pipeline_free(Pipeline& P) {
   P = Pipeline();
 }
 
-// d_points: device buffer holding (resident) or receiving (h_points != nullptr) the n points
-// c_force = 0: window width from n; otherwise the given width (all shards of a multi-device call must share
-// one window plan).  h_partials != nullptr: stop after the bucket reduction and return the W window partials
-// (host copy) instead of the finalized point.
-static int pipeline_run(Pipeline& P, void* d_points, const uint64_t* h_points, const uint64_t* h_scalars, size_t n,
-                        uint64_t* out_jac, int c_force = 0, void* h_partials = nullptr) {
-  CurveInfo ci;
-  curve_info(P.curve, &ci);
-  const size_t sb = (size_t)ci.scalar_bytes;
-  const size_t ab = 8u * ci.coord_words, xb = 16u * ci.coord_words, jb = 12u * ci.coord_words;
-  CK(cudaSetDevice(P.device));
+// batches of a pipelined call over n inputs: batch k is [bstart[k], bstart[k+1]), returns their number.  resident: the points
+// are already on the device (only the scalars cross PCIe).
+static int plan_batches(size_t n, bool resident, size_t bstart[17]) {
   // batch sizes grow geometrically (1/16, 1/8, 3/16, 1/4, 3/8 of n): the first copy is short, and since the
   // GPU consumes a batch more slowly than PCIe delivers the next, every later copy hides under compute
   static const int FR5[5] = {1, 2, 3, 4, 6};   // sixteenths
-  const uint64_t* hp_in = h_points;
   int nch = (n >= (1u << 21)) ? 5 : ((n >= (1u << 18)) ? 2 : 1);
   if (const char* e = getenv("GMSM_CHUNKS")) { int v = atoi(e); if (v >= 1 && v <= 16) nch = v; }
   if ((size_t)nch > n) nch = 1;
   // GMSM_SCHEDULE="1,2,3,5,8": explicit batch weights (experiments; overrides the counts above for n >= 2^18)
   int wts[16], wsum = 0, nw = 0;
-  if (!hp_in && n >= (1u << 21) && !getenv("GMSM_CHUNKS")) {
+  if (resident && n >= (1u << 21) && !getenv("GMSM_CHUNKS")) {
     // resident bases: only the scalars (32 B each) cross PCIe, a third of the one-shot volume, so three batches are
     // enough to hide the copies and every batch less saves its bucket merge + carry join (~1.1 ms each; measured
     // profiles/r01_e2e_schedule_sweep_v15.txt: 4 batches 51.3 ms, 5 batches 52.2 ms at bn254 G1 2^24)
@@ -714,22 +716,45 @@ static int pipeline_run(Pipeline& P, void* d_points, const uint64_t* h_points, c
       if (nw >= 1) nch = nw;
     }
   }
-  size_t bstart[17];
   bstart[0] = 0;
   for (int k = 1; k <= nch; k++) {
     if (nw >= 1) { long acc = 0; for (int u = 0; u < k; u++) acc += wts[u]; bstart[k] = (k == nch) ? n : (size_t)((double)n * acc / wsum); }
     else if (nch == 5) { int acc16 = 0; for (int u = 0; u < k; u++) acc16 += FR5[u]; bstart[k] = (k == nch) ? n : (n / 16) * acc16; }
     else bstart[k] = (k == nch) ? n : (n / nch) * k;
   }
+  return nch;
+}
+static size_t largest_batch(const size_t bstart[17], int nch) {
   size_t nc = 0;
   for (int k = 0; k < nch; k++) nc = std::max(nc, bstart[k + 1] - bstart[k]);
+  return nc;
+}
+static size_t largest_batch(size_t n, bool resident) {
+  size_t bstart[17];
+  return largest_batch(bstart, plan_batches(n, resident, bstart));
+}
+
+// d_points: device buffer holding (resident) or receiving (h_points != nullptr) the n points
+// c_force = 0: window width from n; otherwise the given width (all shards of a multi-device call must share
+// one window plan).  h_partials != nullptr: stop after the bucket reduction and return the W window partials
+// (host copy) instead of the finalized point.
+static int pipeline_run(Pipeline& P, void* d_points, const uint64_t* h_points, const uint64_t* h_scalars, size_t n,
+                        uint64_t* out_jac, int c_force = 0, void* h_partials = nullptr) {
+  CurveInfo ci;
+  curve_info(P.curve, &ci);
+  const size_t sb = (size_t)ci.scalar_bytes;
+  const size_t ab = 8u * ci.coord_words, xb = 16u * ci.coord_words, jb = 12u * ci.coord_words;
+  CK(cudaSetDevice(P.device));
+  size_t bstart[17];
+  const int nch = plan_batches(n, h_points == nullptr, bstart);
+  const size_t nc = largest_batch(bstart, nch);
   if (P.scal_cap < n || P.scal_cap > 4 * n + 1024) {
     cudaFree(P.d_scalars); P.d_scalars = nullptr; P.scal_cap = 0;
     CK(cudaMalloc(&P.d_scalars, n * (size_t)ci.scalar_bytes));
     P.scal_cap = n;
   }
   // window width from the TOTAL size (all batches share one bucket array); workspace sized for one batch
-  const int c = P.tables ? P.tab_c : (c_force ? c_force : choose_c_for(P.curve, ci.fr_bits, n));
+  const int c = P.tables ? P.tab_c : (c_force ? c_force : choose_c_for(P.curve, ci.fr_bits, n, nc));
   if (!P.ctx || P.ctx->max_n < nc || P.ctx->max_n > 4 * nc + 1024 || P.ctx->plan.c != c || P.ctx->shared != P.tables) {
     if (P.ctx) { gmsm_ctx_destroy(P.ctx); P.ctx = nullptr; }
     P.ctx = ctx_create_ex((gmsm_curve_t)P.curve, nc, c, P.device, P.tables);
@@ -1019,7 +1044,8 @@ extern "C" int gmsm_bases_multiexp(gmsm_bases_t* b, size_t offset, const uint64_
   const bool tables = jobs[0].sh->pipe.tables;
   size_t largest = 0;
   for (const auto& j : jobs) largest = std::max(largest, (size_t)(j.e - j.a));
-  const int c = tables ? jobs[0].sh->pipe.tab_c : choose_c_for(b->curve, ci.fr_bits, largest);   // the plan of the largest shard, on all of them
+  // the plan of the largest shard, on all of them
+  const int c = tables ? jobs[0].sh->pipe.tab_c : choose_c_for(b->curve, ci.fr_bits, largest, largest_batch(largest, true));
   const WindowPlan plan = make_plan(ci.fr_bits, c);
   const size_t npart = tables ? 1 : (size_t)plan.nwin;
   std::vector<unsigned char> h_part(jobs.size() * npart * xb);
@@ -1061,7 +1087,7 @@ extern "C" int gmsm_bases_multiexp_device(gmsm_bases_t* b, size_t offset, const 
   BaseShard& sh = b->shards[0];
   Pipeline& P = sh.pipe;
   CK(cudaSetDevice(P.device));
-  const int c = P.tables ? P.tab_c : choose_c_for(P.curve, ci.fr_bits, n);
+  const int c = P.tables ? P.tab_c : choose_c_for(P.curve, ci.fr_bits, n, n);
   if (!P.ctx || P.ctx->max_n < n || P.ctx->max_n > 4 * n + 1024 || P.ctx->plan.c != c || P.ctx->shared != P.tables) {
     if (P.ctx) { gmsm_ctx_destroy(P.ctx); P.ctx = nullptr; }
     P.ctx = ctx_create_ex((gmsm_curve_t)P.curve, n, c, P.device, P.tables);
@@ -1145,7 +1171,7 @@ static int session_prepare(Session& S, int curve, int device, size_t cnt) {
 extern "C" int gmsm_choose_window_bits(gmsm_curve_t curve, size_t n_total) {
   CurveInfo ci;
   if (!curve_info(curve, &ci)) return 0;
-  return choose_c_for(curve, ci.fr_bits, n_total);
+  return choose_c_for(curve, ci.fr_bits, n_total, n_total);
 }
 
 // one shard of a sharded call, host buffers in, W window partials (host) out: the pipelined engine of
@@ -1189,7 +1215,8 @@ extern "C" int gmsm_multiexp(gmsm_curve_t curve, const uint64_t* points, const u
   }
   // ---- multi-device: contiguous shards (the reference's recursive halving, multiexp.go:128-140) ----
   // one plan for every shard (their partials are added window by window), sized for the work ONE device does: the largest shard
-  const int c = choose_c_for(curve, ci.fr_bits, (n + D - 1) / D);
+  const size_t shard = (n + D - 1) / D;
+  const int c = choose_c_for(curve, ci.fr_bits, shard, largest_batch(shard, false));
   const WindowPlan plan = make_plan(ci.fr_bits, c);
   const size_t xb = 16u * ci.coord_words;
   std::vector<unsigned char> h_part(D * plan.nwin * xb);

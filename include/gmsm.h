@@ -101,7 +101,8 @@ int gmsm_multiexp(gmsm_curve_t curve, const uint64_t* points, const uint64_t* sc
                   int nb_tasks, uint64_t* out_jac);
 /* sharded calls with one process per GPU: every process runs its shard through the pipelined engine and gets the W
  * window partials back (host memory, W * gmsm_xyzz_bytes); the partials of all shards are then joined with
- * gmsm_ctx_finalize_device.  All shards must pass the same window width (gmsm_choose_window_bits of the TOTAL size). */
+ * gmsm_ctx_finalize_device.  All shards must pass the same window width (gmsm_choose_window_bits of the TOTAL size).
+ * The width returned keeps n_total * W below 2^32 - 296, the context's 32-bit entry limit, whenever some c <= 24 does. */
 int gmsm_choose_window_bits(gmsm_curve_t curve, size_t n_total);
 int gmsm_multiexp_window_sums(gmsm_curve_t curve, const uint64_t* points, const uint64_t* scalars, size_t n, int c,
                               int device, void* out_partials);
